@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- LU GFLOP/s (FP64, (2/3)N^3) of the CONFLUX hot path on 1/2/4/8 B200 (BASELINE.json's metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...     (N > 1: one rank per GPU)
 
 A "step" is one LU factorisation of one synthetic matrix (lu_params::InitMatrix generator, seed 42):
@@ -14,6 +14,8 @@ A "step" is one LU factorisation of one synthetic matrix (lu_params::InitMatrix 
 memory and the device->host read of the permutation inside the timed region (streamed: the upload of the next
 matrix overlaps the current factorisation; `e2e.single_shot` is the un-overlapped latency of one call).  PyTorch is plumbing only
 (torch.distributed bootstrap, pinned host memory).
+`--dump-outputs DIR` writes, after the timed steps, what the last one handed its caller (see dump_outputs()), so that
+two builds can be compared output for output on the same seeded input.
 """
 import argparse
 import ctypes
@@ -230,6 +232,25 @@ def load_traffic(M, N, K, kernel="dmma"):
     return None, None
 
 
+DUMP_FACTOR_BYTES = 48 << 20     # --dump-outputs: sampled factor rows over all ranks (the whole dump stays under 64 MB)
+
+
+def dump_outputs(dirname, rank, n_holders, factor=None, factor_name=None, perm=None):
+    """--dump-outputs: writes DIR/<name>.npy in float64.  `perm` (the pivot sequence, identical on every rank) goes to
+    lu_perm.npy from rank 0; `factor` (this rank's Ml x Nl block of the factors, None on ranks that hold none) is too
+    large to write whole, so a fixed seeded set of its rows goes to <factor_name>_r<rank>.npy and their local indices to
+    <factor_name>_rows_r<rank>.npy.  The n_holders ranks that hold factors share DUMP_FACTOR_BYTES."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    if perm is not None and rank == 0:
+        np.save(os.path.join(dirname, "lu_perm.npy"), perm.astype(np.float64))
+    if factor is not None:
+        n = max(1, min(factor.shape[0], DUMP_FACTOR_BYTES // (n_holders * factor.shape[1] * 8)))
+        rows = np.sort(np.random.default_rng(rank).choice(factor.shape[0], size=n, replace=False))
+        np.save(os.path.join(dirname, f"{factor_name}_r{rank}.npy"), factor[rows])
+        np.save(os.path.join(dirname, f"{factor_name}_rows_r{rank}.npy"), rows.astype(np.float64))
+
+
 CHOL_WORKLOAD = (32768, 512)     # BASELINE.json configs[4]: cholesky_miniapp --dim=32768 --tile=512 (8 x B200)
 
 
@@ -293,6 +314,8 @@ def run_cholesky(args, rank, world, local_rank):
         ch.parallelCholesky(upload=True)
     barrier()
     e2e_ms = max_over_ranks((time.perf_counter() - t0) * 1e3) / args.steps
+    if args.dump_outputs:       # the factor of the last timed step; only layer 0 holds it
+        dump_outputs(args.dump_outputs, rank, ch.PX * ch.PY, ch.local_factor() if ch.pz == 0 else None, "chol_factor")
     resid_abs, resid = ch.validate()
     if rank == 0:
         grid = (ch.PX, ch.PY, ch.PZ)
@@ -340,7 +363,12 @@ def main():
     ap.add_argument("--v", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-validate", action="store_true", help="skip the grid-wide residual (debugging only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computes; --impl reference has no outputs to write")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -455,6 +483,12 @@ def main():
     barrier()
     e2e1_ms = max_over_ranks((time.perf_counter() - t0) * 1e3) / args.steps
     e2e1_val = flops / (e2e1_ms * 1e-3) / 1e9
+    if args.dump_outputs:       # what LU_rep(gv, C, perm) hands over after the last timed step; only layer 0 holds factors
+        C = None
+        if gv.pk == 0:
+            C = np.empty((gv.Ml, gv.Nl))
+            _lib.check(L.cflx_lu_get_factors(gv._h, C.ctypes.data, None), "lu_get_factors")
+        dump_outputs(args.dump_outputs, rank, Px * Py, C, "lu_factors", perm)
 
     # ---- parity of the run that was just timed (every rank takes part: the residual is a grid collective) ------------
     ok_perm = sorted(perm.tolist()) == list(range(gv.M))

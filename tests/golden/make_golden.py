@@ -1,6 +1,7 @@
 """tests/golden/make_golden.py -- regenerates tests/golden/*.npz by running THE REFERENCE ITSELF
 (oracle/_ref/libref_lu.so = /root/reference sources compiled by oracle/build_ref.sh; ranks are threads).
 Run in the build container only (needs /root/reference):  python tests/golden/make_golden.py
+    [helpers] [lu_cases] [lu_ref_cases] [layouts]   (default: all)
 
 Fixtures:
   helpers.npz  - the reference's building blocks on the inputs of its own unit test
@@ -9,10 +10,18 @@ Fixtures:
   lu_cases.npz - full LU_rep outputs (input A, C, permutation) on small grids, incl. the hard-coded
                  matrices of lu_params.hpp:157-363 (N = 16, 27, 32) and multi-rank / multi-layer grids.
   lu_perms.npz - permutation-only known answers for larger seeded inputs (N = 256, 1024, 2048).
+  lu_ref_cases.npz - LU_rep on the grids of tests/test_oracle_vs_reference.py: a SHA-256 digest of the generated
+                 input, the permutation and a seeded sample of the factors (the full factors would exceed 1 MB).
+  layouts.txt  - the reference's conflux_layout / lu_params::matrix COSTA descriptors (tests/cpp/layout_ref_dump.cpp,
+                 compiled against the sources under $CONFLUX_REFERENCE), for tests/test_layout_vs_costa.py.
 """
 import ctypes
+import hashlib
 import os
+import subprocess
 import sys
+import sysconfig
+import tempfile
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -104,9 +113,47 @@ def lu_cases():
     np.savez_compressed(os.path.join(HERE, "lu_perms.npz"), **perms)
 
 
+REF_CASES = [(48, 4, 1, 1, 1), (128, 16, 2, 2, 1), (128, 8, 2, 2, 2), (96, 16, 1, 1, 2), (72, 4, 3, 3, 2), (256, 32, 4, 4, 1)]
+REF_SAMPLE = 1024        # factor entries kept per case
+
+
+def lu_ref_cases():
+    out = {"cases": np.array(REF_CASES, dtype=np.int32)}
+    for i, (N, v, Px, Py, Pz) in enumerate(REF_CASES):
+        r = ref.lu_run(N, v, Px, Py, Pz)
+        out[f"c{i}_A_sha256"] = np.array(hashlib.sha256(np.ascontiguousarray(np.stack(r["A"])).tobytes()).hexdigest())
+        out[f"c{i}_perm"] = r["perm"]
+        C = np.stack(r["C"]).reshape(-1)
+        idx = np.sort(np.random.default_rng(i).choice(C.size, size=min(REF_SAMPLE, C.size), replace=False))
+        out[f"c{i}_C_idx"] = idx.astype(np.int32)
+        out[f"c{i}_C_val"] = C[idx]
+    np.savez_compressed(os.path.join(HERE, "lu_ref_cases.npz"), **out)
+
+
+def layouts():
+    src = os.environ.get("CONFLUX_REFERENCE")
+    if not src or not os.path.isdir(os.path.join(src, "libs", "costa", "src")):
+        sys.exit("layouts: set CONFLUX_REFERENCE to the reference checkout (eth-cscs/conflux with libs/costa)")
+    costa = os.path.join(src, "libs", "costa", "src")
+    sp = sysconfig.get_paths()["purelib"]
+    libs = os.path.join(sp, "opencv_python_headless.libs")
+    blas = os.path.join(libs, sorted(f for f in os.listdir(libs) if f.startswith("libopenblasp"))[0])
+    with tempfile.TemporaryDirectory() as tmp:
+        exe = os.path.join(tmp, "layout_ref_dump")
+        srcs = [f"{src}/src/conflux/lu/layout.cpp", f"{costa}/costa/layout.cpp", f"{ROOT}/oracle/mpi_stub/mpi_threads.cpp"] + \
+               [f"{costa}/costa/grid2grid/{f}.cpp" for f in ("block", "grid2D", "interval", "scalapack_layout", "ranks_reordering")]
+        subprocess.check_call(["g++", "-O1", "-std=c++17", "-fopenmp", "-w", "-DNDEBUG", f"-I{ROOT}/oracle/mpi_stub", f"-I{costa}",
+                               f"-I{src}/src", f"{ROOT}/tests/cpp/layout_ref_dump.cpp"] + srcs +
+                              [blas, f"-Wl,-rpath,{libs}", f"-Wl,-rpath,{sp}/scipy.libs", "-lpthread", "-o", exe])
+        txt = subprocess.run([exe], capture_output=True, text=True, check=True).stdout
+    with open(os.path.join(HERE, "layouts.txt"), "w") as f:
+        f.write(txt)
+
+
 if __name__ == "__main__":
     if not ref.available():
         sys.exit("oracle/_ref/libref_lu.so missing: run oracle/build_ref.sh in the build container first")
-    helpers()
-    lu_cases()
+    steps = {"helpers": helpers, "lu_cases": lu_cases, "lu_ref_cases": lu_ref_cases, "layouts": layouts}
+    for name in [a for a in sys.argv[1:] if a in steps] or list(steps):
+        steps[name]()
     print("golden fixtures written to", HERE)
