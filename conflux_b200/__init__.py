@@ -5,6 +5,7 @@ error behaviour; reference file:line relative to eth-cscs/conflux):
 
     lu_params(M, N, v[, Px, Py, Pz], comm)   src/conflux/lu/lu_params.hpp:401-409   sizes, grid, InitMatrix, data
     LU_rep(params, C, permutation) -> ms      src/conflux/lu/conflux_opt.hpp:343-346 the factorisation
+    LU_solve(params, B_local) -> (X, ms)      (no counterpart in the reference) A X = B with those factors
 
 All arithmetic happens in libconflux_b200.so (hand-written CUDA, include/conflux_b200.h is the C ABI);
 this package is a thin ctypes host layer and never falls back to a CPU path.
@@ -15,7 +16,7 @@ import numpy as np
 
 from ._lib import ConfluxError, LIB_PATH, SYMBOLS, check, lib
 
-__all__ = ["pinned_empty", "pinned_free", "Comm", "lu_params", "LU_rep", "residual", "validate", "timeline", "auto_grid", "lu_dims", "init_matrix_host", "ConfluxError", "dbg", "cholesky", "chol_dims", "chol_auto_grid"]
+__all__ = ["pinned_empty", "pinned_free", "Comm", "lu_params", "LU_rep", "LU_solve", "residual", "validate", "timeline", "auto_grid", "lu_dims", "init_matrix_host", "ConfluxError", "dbg", "cholesky", "chol_dims", "chol_auto_grid"]
 
 
 def auto_grid(M, N, P):
@@ -178,6 +179,32 @@ def LU_rep(gv, C=None, permutation=None, upload=True, next_data=None):
     return ms.value
 
 
+def LU_solve(gv, B_local, nrhs=None):
+    """Solves A X = B with the factors of the last LU_rep (P A = L U, A the padded M x M matrix).  COLLECTIVE over
+    gv.lu_comm, with the same number of right-hand sides on every rank.
+
+    B_local: this rank's rows of B in A's row distribution, (Ml, nrhs) float64 C-contiguous (or (Ml,) for one
+    right-hand side): global row g on grid row (g // v) % Px at local row (g // (v*Px))*v + g % v.  It is read on the
+    ranks with pj == 0 and pk == 0; elsewhere it may be None, and then nrhs must be given.
+    Returns (X_local, ms): X_local (Nl, nrhs) (or (Nl,)) holds X in A's column distribution -- global row g on every rank
+    with pj == (g // v) % Py at local row (g // (v*Py))*v + g % v -- and ms is the device time of the solve proper."""
+    vector = False
+    if B_local is not None:
+        assert B_local.dtype == np.float64 and B_local.flags.c_contiguous and B_local.ndim in (1, 2) \
+            and B_local.shape[0] == gv.Ml
+        vector = B_local.ndim == 1
+        n = 1 if vector else B_local.shape[1]
+        assert nrhs is None or nrhs == n
+        nrhs = n
+    if nrhs is None or nrhs < 1:
+        raise ValueError("LU_solve: nrhs >= 1 is needed when B_local is None")
+    X = np.empty((gv.Nl,) if vector else (gv.Nl, int(nrhs)), dtype=np.float64)
+    ms = ctypes.c_double()
+    check(lib().cflx_lu_solve(gv._h, int(nrhs), B_local.ctypes.data if B_local is not None else None, X.ctypes.data,
+                              ctypes.byref(ms)), "lu_solve")
+    return X, ms.value
+
+
 def timeline(gv):
     """Per-region device time of the last LU_rep run under cflx_lu_set_profiling(gv._h, 1 or 2): dict(main={region: (ms,
     count)}, side={...}); region names are the reference's semiprof regions."""
@@ -316,6 +343,16 @@ class dbg:
                                   X.ctypes.data if X is not None else None, R.ctypes.data if R is not None else None,
                                   Y.ctypes.data if Y is not None else None), "dbg_trsm")
         return X, Y
+
+    @staticmethod
+    def trsm_left_upper(A00, R):
+        """X = U^-1 R with U = upper(A00) (v x v) and R (v x n): the diagonal-tile solve of LU_solve."""
+        A00 = np.ascontiguousarray(A00, dtype=np.float64)
+        R = np.ascontiguousarray(R, dtype=np.float64)
+        v, n = R.shape
+        X = np.empty_like(R)
+        check(lib().cflx_dbg_trsm_left_upper(v, n, A00.ctypes.data, R.ctypes.data, X.ctypes.data), "dbg_trsm_left_upper")
+        return X
 
     @staticmethod
     def ozaki_gemm(AT, B, C=None, reps=1, want_planes=False):

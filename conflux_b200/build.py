@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libconflux_b200.so")
-SOURCES = ["gemm.cu", "ozaki.cu", "panel.cu", "rows.cu", "trsm.cu", "lu.cu", "validate.cu", "chol.cu", "dbg.cu"]
+SOURCES = ["gemm.cu", "ozaki.cu", "panel.cu", "rows.cu", "trsm.cu", "lu.cu", "validate.cu", "solve.cu", "chol.cu", "dbg.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC,-O3",
          "-ccbin", "g++", "--expt-relaxed-constexpr"]

@@ -255,6 +255,37 @@ int cflx_dbg_trsm(int n, int v, const double* A00, const double* B, double* X_ou
     return CFLX_OK;
 }
 
+// the diagonal-tile solve of cflx_lu_solve: X = U^-1 R with the transposed block inverses of diag_inverse_kernel
+int cflx_dbg_trsm_left_upper(int v, int n, const double* A00, const double* R, double* X_out) {
+    CFLX_TRY(check_device());
+    if (n <= 0 || v <= 0 || v % 4 != 0 || !A00 || !R || !X_out) return CFLX_ERR_ARG;
+    int nb = 0;
+    for (int c : {128, 64, 32, 16, 8, 4})
+        if (!nb && v % c == 0) nb = c;
+    if (nb == 0) return CFLX_ERR_UNSUPPORTED;
+    const int64_t ld = round_up(n, 2);
+    std::vector<double> A00T((size_t)v * v), RT((size_t)v * ld, 0.0);
+    for (int i = 0; i < v; ++i)
+        for (int j = 0; j < v; ++j) A00T[(size_t)j * v + i] = A00[(size_t)i * v + j];
+    for (int i = 0; i < v; ++i)
+        for (int c = 0; c < n; ++c) RT[(size_t)i * ld + c] = R[(size_t)i * n + c];
+    DevBuf dA, dAT, dUinvT, dLinvT, dR, dX;
+    CFLX_TRY(dA.alloc(8 * (size_t)v * v)); CFLX_TRY(dAT.alloc(8 * (size_t)v * v));
+    CFLX_TRY(dUinvT.alloc(8 * (size_t)v * v)); CFLX_TRY(dLinvT.alloc(8 * (size_t)v * v));
+    CFLX_TRY(dR.alloc(8 * (size_t)v * ld)); CFLX_TRY(dX.alloc(8 * (size_t)v * ld));
+    CFLX_CUDA(cudaMemcpy(dA.p, A00, 8 * (size_t)v * v, cudaMemcpyHostToDevice));
+    CFLX_CUDA(cudaMemcpy(dAT.p, A00T.data(), 8 * (size_t)v * v, cudaMemcpyHostToDevice));
+    CFLX_CUDA(cudaMemcpy(dR.p, RT.data(), 8 * (size_t)v * ld, cudaMemcpyHostToDevice));
+    CFLX_CUDA(cudaMemset(dX.p, 0, 8 * (size_t)v * ld));
+    CFLX_TRY(launch_diag_inverses(dA.as<double>(), v, nb, dUinvT.as<double>(), dLinvT.as<double>(), 0, true));
+    CFLX_TRY(trsm_left_upper(dAT.as<double>(), dUinvT.as<double>(), v, nb, dR.as<double>(), dX.as<double>(), ld, (int)ld, 0));
+    CFLX_CUDA(cudaMemcpy(RT.data(), dX.p, 8 * (size_t)v * ld, cudaMemcpyDeviceToHost));
+    for (int i = 0; i < v; ++i)
+        for (int c = 0; c < n; ++c) X_out[(size_t)i * n + c] = RT[(size_t)i * ld + c];
+    CFLX_CUDA(cudaDeviceSynchronize());
+    return CFLX_OK;
+}
+
 // step 2 of the LU loop in isolation on ONE rank (Px = 1): plan_moves (analyze_pivots) + push_phase1..3 (push_pivots_up,
 // conflux_opt.hpp:176-218) + the gri/igri bookkeeping, on an n_rows x n_cols row-major matrix (n_cols even).  The npiv
 // pivot rows (local indices >= fnpr, tournament order) end up in rows [fnpr, fnpr+npiv) in that order.

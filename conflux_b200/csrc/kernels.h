@@ -126,13 +126,26 @@ int launch_unpack_bcast(const double* buf, int v, double* A00, double* A00T, int
 int launch_record_pivots(const int* gpivots, int v, int* hist, int k, cudaStream_t stream);
 
 // ---------------------------------------------------------------- trsm.cu
-// inverses of the nb x nb diagonal blocks of A00 = L00\U00: Uinv[j] (row-major) and LinvT[j] (= inv(L_jj)^T)
-int launch_diag_inverses(const double* A00, int v, int nb, double* Uinv, double* LinvT, cudaStream_t stream);
+// inverses of the nb x nb diagonal blocks of A00 = L00\U00: Uinv[j] (row-major; inv(U_jj)^T when u_transposed) and
+// LinvT[j] (= inv(L_jj)^T)
+int launch_diag_inverses(const double* A00, int v, int nb, double* Uinv, double* LinvT, cudaStream_t stream,
+                         bool u_transposed = false);
 // LT = (PT * U00^-1)^T : PT, LT are [v][ld] transposed panels with n columns; PT is destroyed
 int trsm_right_upper_T(const double* A00, const double* Uinv, int v, int nb, double* PT, double* LT, int64_t ld,
                        int n, cudaStream_t stream);
 // U = L00^-1 * R : R, U are [v][ld] with n columns; R is destroyed
 int trsm_left_lower_unit(const double* A00T, const double* LinvT, int v, int nb, double* R, double* U, int64_t ld,
                          int n, cudaStream_t stream);
+// X = U00^-1 * R (left, upper, non-unit) : R, X are [v][ld] with n columns (n even); R is destroyed.  A00T = U00^T
+// (lower part ignored), UinvT = the transposed diagonal-block inverses (launch_diag_inverses, u_transposed)
+int trsm_left_upper(const double* A00T, const double* UinvT, int v, int nb, double* R, double* X, int64_t ld, int n,
+                    cudaStream_t stream);
+
+// ---------------------------------------------------------------- solve.cu
+// W[r][c] -= sum_k AT[k][r] * Y[k][c] for r < M, c < n (n <= 16): the few-right-hand-side trailing update of the
+// distributed triangular solves, bandwidth-bound on the AT panel (K = v rows of ldat doubles)
+int launch_solve_update_skinny(const double* AT, int64_t ldat, int M, int K, const double* Y, int64_t ldy, int n,
+                               double* W, int64_t ldw, cudaStream_t stream);
+constexpr int SOLVE_SKINNY_MAX = 16;  // widest right-hand-side block of the skinny update
 
 }  // namespace cflx

@@ -514,6 +514,7 @@ void free_lu(cflx_lu* lu) {
     if (lu->copy) cudaStreamDestroy(lu->copy);
     if (lu->ev_a0_read) cudaEventDestroy(lu->ev_a0_read);
     if (lu->ev_upload) cudaEventDestroy(lu->ev_upload);
+    solve_state_free(&lu->sv);
     for (SubComm* sc : {&lu->k_comm, &lu->i_comm, &lu->jk_comm, &lu->ik_comm})
         if (sc->c) ncclCommDestroy(sc->c);
     delete lu;
@@ -790,6 +791,7 @@ int cflx_lu_set_local(cflx_lu* lu, const double* host_local) {
     CFLX_CUDA(cudaStreamSynchronize(lu->comm->stream));
     lu->have_input = true;
     lu->factored = false;
+    lu->sv.ready = false;
     lu->a0_is_next = false;
     lu->next_host = nullptr;
     return CFLX_OK;
@@ -821,6 +823,7 @@ int cflx_lu_factor(cflx_lu* lu, double* ms_out) {
         set_last_error("cflx_lu_factor before cflx_lu_set_local");
         return CFLX_ERR_STATE;
     }
+    lu->sv.ready = false;  // the solve's copy of the factors describes the previous factorisation
     cflx_comm* c = lu->comm;
     cudaStream_t s = c->stream;
     CFLX_CUDA(cudaSetDevice(c->device));

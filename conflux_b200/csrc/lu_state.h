@@ -61,6 +61,18 @@ inline int dmalloc(T** p, size_t n) {
 }
 int make_sub(cflx_comm* c, int color, int key, int size, SubComm* out);
 int grid_barrier(cflx_comm* c);
+
+// State of cflx_lu_solve (solve.cu): the factors re-laid out for the triangular sweeps, built on the first solve after
+// each factorisation, and the right-hand-side work buffers, grown to the widest solve so far.
+struct SolveState {
+    bool ready = false;             // CT / diagonal blocks describe the current factors
+    std::vector<int> hist;          // pivot history of those factors (row of global id hist[q] is pivoted row q)
+    std::vector<int> diag_slot;     // [Nt] index of diagonal tile t among this rank's diagonal tiles, -1 if not mine
+    double* CT = nullptr;           // [Nl][Ml] (layer 0): CT[lc][r] = C[r][lc], C the factors in the conflux layout
+    double* diag = nullptr;         // per owned diagonal tile: DT [v][v] (transposed tile), LinvT [v*nb], UinvT [v*nb]
+    double *W = nullptr, *X = nullptr, *B = nullptr, *stage = nullptr;  // Ml x ldr, Nl x ldr, Ml x ldr, 2 Ml x ldr
+    int ldr_cap = 0;
+};
 }  // namespace cflx
 
 struct cflx_lu {
@@ -101,10 +113,15 @@ struct cflx_lu {
     std::vector<char> ev_used;
     cudaStream_t side = nullptr;  // high-priority look-ahead stream (null: no overlap)
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_npiv = nullptr;
+    cflx::SolveState sv;  // cflx_lu_solve (marked stale by cflx_lu_set_local / cflx_lu_factor)
 };
 
 namespace cflx {
 // validate.cu
 int redistribute_pivoted_rows(cflx_lu* lu, const std::vector<int>& hist, bool factors, const double* src, double* dst);
+int redistribute_pivoted_rows(cflx_lu* lu, const std::vector<int>& hist, bool factors, const double* src, double* dst,
+                              int ncols, int64_t ld, double* stage);
 int lu_residual_grid(cflx_lu* lu, const std::vector<int>& hist, double* abs_out, double* rel_out);
+// solve.cu
+void solve_state_free(SolveState* sv);
 }  // namespace cflx

@@ -12,14 +12,15 @@
 
 namespace cflx {
 namespace {
-// grid = (nblk, 2, CS): y == 0 -> Uinv[j] = inv(U_jj) row-major; y == 1 -> LinvT[j] = inv(L_jj)^T row-major; the columns of
-// a block are split over CS = gridDim.z CTAs (each stages the whole block in shared memory).
+// grid = (nblk, 2, CS): y == 0 -> Uinv[j] = inv(U_jj) row-major (u_transposed: inv(U_jj)^T, the operand of the left
+// upper solve); y == 1 -> LinvT[j] = inv(L_jj)^T row-major; the columns of a block are split over CS = gridDim.z CTAs
+// (each stages the whole block in shared memory).
 // One WARP per column of the inverse: the column lives in registers spread over the lanes (lane l holds entries l, l + 32,
 // ...), every substitution step is a short partial dot product per lane + a warp reduction, so an NB x NB block takes NB
 // steps of ~100 cycles per column instead of an NB^2 / 2 serial FMA chain per thread.
 template <int NB>
 __global__ void __launch_bounds__(1024) diag_inverse_kernel(const double* __restrict__ A00, int v, double* __restrict__ Uinv,
-                                                            double* __restrict__ LinvT) {
+                                                            double* __restrict__ LinvT, int u_transposed) {
     constexpr int EPL = (NB + 31) / 32;  // entries per lane
     extern __shared__ double S[];        // [NB][NB + 1]
     constexpr int LD = NB + 1;
@@ -57,7 +58,7 @@ __global__ void __launch_bounds__(1024) diag_inverse_kernel(const double* __rest
 #pragma unroll
             for (int e = 0; e < EPL; ++e) {
                 const int t = lane + 32 * e;
-                if (t < NB) out[(size_t)t * NB + c] = x[e];  // Uinv[r][c]
+                if (t < NB) out[u_transposed ? (size_t)c * NB + t : (size_t)t * NB + c] = x[e];  // Uinv[t][c]
             }
         } else {  // L Y = I (unit diagonal): y[c] = 1; y[r] = -sum_{t=c..r-1} L[r][t] y[t], r > c
 #pragma unroll
@@ -86,27 +87,28 @@ __global__ void __launch_bounds__(1024) diag_inverse_kernel(const double* __rest
 }
 
 template <int NB>
-int launch_diag_nb(const double* A00, int v, double* Uinv, double* LinvT, cudaStream_t stream) {
+int launch_diag_nb(const double* A00, int v, double* Uinv, double* LinvT, bool u_transposed, cudaStream_t stream) {
     constexpr size_t smem = (size_t)NB * (NB + 1) * sizeof(double);
     constexpr int CS = NB > 64 ? NB / 32 : 1;   // 128-wide blocks: 4 CTAs x 32 columns, one column per warp
     const int warps = NB < 32 ? NB : 32;
     static PerDeviceMax cfg;
     if (cfg.raise(smem))
         CFLX_CUDA(cudaFuncSetAttribute(diag_inverse_kernel<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    diag_inverse_kernel<NB><<<dim3(v / NB, 2, CS), 32 * warps, smem, stream>>>(A00, v, Uinv, LinvT);
+    diag_inverse_kernel<NB><<<dim3(v / NB, 2, CS), 32 * warps, smem, stream>>>(A00, v, Uinv, LinvT, u_transposed ? 1 : 0);
     CFLX_CUDA(cudaGetLastError());
     return CFLX_OK;
 }
 }  // namespace
 
-int launch_diag_inverses(const double* A00, int v, int nb, double* Uinv, double* LinvT, cudaStream_t stream) {
+int launch_diag_inverses(const double* A00, int v, int nb, double* Uinv, double* LinvT, cudaStream_t stream,
+                         bool u_transposed) {
     switch (nb) {
-        case 128: return launch_diag_nb<128>(A00, v, Uinv, LinvT, stream);
-        case 64: return launch_diag_nb<64>(A00, v, Uinv, LinvT, stream);
-        case 32: return launch_diag_nb<32>(A00, v, Uinv, LinvT, stream);
-        case 16: return launch_diag_nb<16>(A00, v, Uinv, LinvT, stream);
-        case 8: return launch_diag_nb<8>(A00, v, Uinv, LinvT, stream);
-        case 4: return launch_diag_nb<4>(A00, v, Uinv, LinvT, stream);
+        case 128: return launch_diag_nb<128>(A00, v, Uinv, LinvT, u_transposed, stream);
+        case 64: return launch_diag_nb<64>(A00, v, Uinv, LinvT, u_transposed, stream);
+        case 32: return launch_diag_nb<32>(A00, v, Uinv, LinvT, u_transposed, stream);
+        case 16: return launch_diag_nb<16>(A00, v, Uinv, LinvT, u_transposed, stream);
+        case 8: return launch_diag_nb<8>(A00, v, Uinv, LinvT, u_transposed, stream);
+        case 4: return launch_diag_nb<4>(A00, v, Uinv, LinvT, u_transposed, stream);
         default:
             set_last_error("diag_inverses: unsupported block size %d", nb);
             return CFLX_ERR_UNSUPPORTED;
@@ -167,6 +169,36 @@ int trsm_left_lower_unit(const double* A00T, const double* LinvT, int v, int nb,
             u.B = U + (int64_t)j * nb * ld; u.ldb = ld;
             u.C = R + (int64_t)(j + 1) * nb * ld; u.ldc = ld;
             u.D = R + (int64_t)(j + 1) * nb * ld; u.ldd = ld;
+            u.alpha = -1.0; u.beta = 1.0;
+            CFLX_TRY(launch_gemm_tn(u, stream));
+        }
+    }
+    return CFLX_OK;
+}
+
+// U00 * X = R (non-unit upper), the bottom-up mirror of trsm_left_lower_unit.  R/X are [v][ld]:
+//   X_j = inv(U_jj) * R_j ;  R_i -= U_ij * X_j  (i < j, all block rows above j in one GEMM)
+// UinvT holds inv(U_jj)^T (launch_diag_inverses with u_transposed), A00T[c][r] = U00[r][c].
+int trsm_left_upper(const double* A00T, const double* UinvT, int v, int nb, double* R, double* X, int64_t ld, int n,
+                    cudaStream_t stream) {
+    if (n <= 0) return CFLX_OK;
+    const int nblk = v / nb;
+    for (int j = nblk - 1; j >= 0; --j) {
+        GemmArgs g{};
+        g.M = nb; g.N = n; g.K = nb;
+        g.AT = UinvT + (size_t)j * nb * nb; g.ldat = nb;             // AT[k][m] = inv(U_jj)[m][k]
+        g.B = R + (int64_t)j * nb * ld; g.ldb = ld;
+        g.C = nullptr; g.ldc = ld;
+        g.D = X + (int64_t)j * nb * ld; g.ldd = ld;
+        g.alpha = 1.0; g.beta = 0.0;
+        CFLX_TRY(launch_gemm_tn(g, stream));
+        if (j > 0) {
+            GemmArgs u{};
+            u.M = j * nb; u.N = n; u.K = nb;
+            u.AT = A00T + (size_t)(j * nb) * v; u.ldat = v;               // AT[k][m] = U[m][j*nb+k]
+            u.B = X + (int64_t)j * nb * ld; u.ldb = ld;
+            u.C = R; u.ldc = ld;
+            u.D = R; u.ldd = ld;
             u.alpha = -1.0; u.beta = 1.0;
             CFLX_TRY(launch_gemm_tn(u, stream));
         }

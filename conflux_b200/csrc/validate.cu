@@ -81,10 +81,18 @@ __global__ void extract_u_block_kernel(const double* __restrict__ C, int64_t ldc
 // promoted row);  otherwise src = the pristine input A0 (row of global id g at its original local slot), i.e. dst = P*A.
 // Collective over the i-communicator of layer 0 (ranks with pk != 0 must not call).
 int redistribute_pivoted_rows(cflx_lu* lu, const std::vector<int>& hist, bool factors, const double* src, double* dst) {
+    if (lu->Px > 1 && !lu->xbuf) CFLX_TRY(dmalloc(&lu->xbuf, 2 * (size_t)lu->Ml * lu->Nl));
+    return redistribute_pivoted_rows(lu, hist, factors, src, dst, lu->Nl, lu->Nl, lu->xbuf);
+}
+
+// The same on rows of `ncols` doubles at leading dimension ld (both even) of src and dst, e.g. the right-hand sides of
+// cflx_lu_solve (factors = false: dst = P*B).  stage: 2 * Ml * ncols doubles of staging, needed when Px > 1.
+int redistribute_pivoted_rows(cflx_lu* lu, const std::vector<int>& hist, bool factors, const double* src, double* dst,
+                              int ncols, int64_t ld, double* stage) {
     cflx_comm* c = lu->comm;
     cudaStream_t s = c->stream;
-    const int v = lu->v, Px = lu->Px, Ml = lu->Ml, Nl = lu->Nl;
-    const size_t loc = (size_t)Ml * Nl;
+    const int v = lu->v, Px = lu->Px, Ml = lu->Ml;
+    const size_t loc = (size_t)Ml * ncols;
     if (!lu->idx_buf) CFLX_TRY(dmalloc(&lu->idx_buf, 2 * (size_t)Ml));
     std::vector<int> next_local(Px, 0);
     std::vector<std::vector<int>> send_rows(Px), recv_rows(Px);  // send_rows[dst rank] = my source rows; recv_rows[src rank] = my dest rows
@@ -111,22 +119,21 @@ int redistribute_pivoted_rows(cflx_lu* lu, const std::vector<int>& hist, bool fa
     }
     CFLX_CUDA(cudaMemcpyAsync(lu->idx_buf, flat_send.data(), sizeof(int) * Ml, cudaMemcpyHostToDevice, s));
     CFLX_CUDA(cudaMemcpyAsync(lu->idx_buf + Ml, flat_recv.data(), sizeof(int) * Ml, cudaMemcpyHostToDevice, s));
-    dim3 grid(std::max(1, std::min(32, Nl / 512)), Ml);
+    dim3 grid(std::max(1, std::min(32, ncols / 512)), Ml);
     if (Px == 1) {
-        move_rows_kernel<<<grid, 256, 0, s>>>(src, Nl, lu->idx_buf, lu->idx_buf + Ml, Ml, Nl, dst, Nl);
+        move_rows_kernel<<<grid, 256, 0, s>>>(src, ld, lu->idx_buf, lu->idx_buf + Ml, Ml, ncols, dst, ld);
         CFLX_CUDA(cudaGetLastError());
         CFLX_CUDA(cudaStreamSynchronize(s));  // the index vectors above are stack/heap temporaries
         return CFLX_OK;
     }
-    if (!lu->xbuf) CFLX_TRY(dmalloc(&lu->xbuf, 2 * loc));
-    double* sendbuf = lu->xbuf;
-    double* recvbuf = lu->xbuf + loc;
-    gather_rows_kernel<<<grid, 256, 0, s>>>(src, Nl, lu->idx_buf, Ml, Nl, sendbuf);
+    double* sendbuf = stage;
+    double* recvbuf = stage + loc;
+    gather_rows_kernel<<<grid, 256, 0, s>>>(src, ld, lu->idx_buf, Ml, ncols, sendbuf);
     CFLX_CUDA(cudaGetLastError());
     CFLX_NCCL(ncclGroupStart());
     size_t so = 0, ro = 0;
     for (int p = 0; p < Px; ++p) {
-        const size_t ns = send_rows[p].size() * (size_t)Nl, nr = recv_rows[p].size() * (size_t)Nl;
+        const size_t ns = send_rows[p].size() * (size_t)ncols, nr = recv_rows[p].size() * (size_t)ncols;
         if (p == lu->pi) {
             CFLX_CUDA(cudaMemcpyAsync(recvbuf + ro, sendbuf + so, ns * sizeof(double), cudaMemcpyDeviceToDevice, s));
         } else {
@@ -137,7 +144,7 @@ int redistribute_pivoted_rows(cflx_lu* lu, const std::vector<int>& hist, bool fa
         ro += nr;
     }
     CFLX_NCCL(ncclGroupEnd());
-    scatter_rows_kernel<<<grid, 256, 0, s>>>(recvbuf, Nl, lu->idx_buf + Ml, Ml, dst, Nl);
+    scatter_rows_kernel<<<grid, 256, 0, s>>>(recvbuf, ncols, lu->idx_buf + Ml, Ml, dst, ld);
     CFLX_CUDA(cudaGetLastError());
     CFLX_CUDA(cudaStreamSynchronize(s));
     return CFLX_OK;

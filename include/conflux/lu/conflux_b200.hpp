@@ -244,6 +244,17 @@ std::size_t LU_rep(lu_params<T>& gv, T* C, int* permutation) {
     return (std::size_t)ms;
 }
 
+// A X = B with the factors of the last LU_rep (no counterpart in the reference).  Collective over gv.lu_comm.
+// B: this rank's Ml x nrhs rows of B in A's row distribution (read on ranks with pj == 0 && pk == 0, may be null
+// elsewhere); X: Nl x nrhs, filled on every rank with X in A's column distribution (cflx_lu_solve in conflux_b200.h).
+// Returns the device time of the solve in ms (truncated like LU_rep).
+template <class T>
+std::size_t LU_solve(lu_params<T>& gv, int nrhs, const T* B, T* X) {
+    double ms = 0;
+    check(cflx_lu_solve(gv.plan, nrhs, B, X, &ms), "LU_solve");
+    return (std::size_t)ms;
+}
+
 // The reference's validation (examples/conflux_miniapp.cpp:349-500) of the last LU_rep, on the GPU grid.  Collective.
 // Returns ||P*A - L*U||_F (what the reference prints as "Total Frobenius norm"); *relative = that / ||A||_F.
 template <class T>

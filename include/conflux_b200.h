@@ -15,6 +15,7 @@
  *   lu_params<T>::data (local tiles, ld = Nl) ........ src/conflux/lu/layout.cpp:95-109      -> cflx_lu_set_local
  *   LU_rep<T>(gv, C, permutation) main loop .......... src/conflux/lu/conflux_opt.hpp:343-1827 -> cflx_lu_factor
  *   validation outputs C / permutation ............... src/conflux/lu/conflux_opt.hpp:1660-1771,1822 -> cflx_lu_get_factors
+ * Beyond the reference: cflx_lu_solve solves A X = B with the factors where they lie, on the same grid.
  * There is no CPU fallback: without a CUDA device every device entry point returns CFLX_ERR_NO_DEVICE.
  */
 #ifndef CONFLUX_B200_H
@@ -95,6 +96,18 @@ int cflx_lu_get_permutation(cflx_lu*, int* permutation_out);
 int cflx_lu_validate(cflx_lu*, double* frob_abs_out, double* frob_rel_out);
 /* COLLECTIVE.  = cflx_lu_validate(lu, NULL, rel_out) */
 int cflx_lu_residual(cflx_lu*, double* rel_out);
+/* COLLECTIVE.  Solves A X = B with the factors of the last cflx_lu_factor (P A = L U, A is the padded M x M matrix),
+ * nrhs >= 1 right-hand sides, the same nrhs on every rank.
+ * B_local: Ml x nrhs, row-major, ld = nrhs -- B in A's ROW distribution: global row g lives on grid row (g / v) % Px
+ *          at local row (g / (v*Px))*v + g % v.  Read on ranks with pj == 0 && pk == 0; ignored (may be NULL) elsewhere.
+ * X_local: Nl x nrhs, row-major -- X in A's COLUMN distribution: global row g on every rank with pj == (g / v) % Py
+ *          (all pi, all pk) at local row (g / (v*Py))*v + g % v.  Written on every rank.
+ * ms_out (may be NULL): device time of the solve proper (grid barrier .. last X tile), excluding the upload of B, the
+ * read-back of X and the one-time preparation after each factorisation.
+ * Does not modify the factors: cflx_lu_get_factors / cflx_lu_validate afterwards return what they returned before.
+ * CFLX_ERR_STATE before any cflx_lu_factor or after a cflx_lu_set_local no factorisation has consumed (a streamed
+ * factorisation, cflx_lu_queue_next_local, keeps its factors solvable).  As in dgetrs, there is no singularity check. */
+int cflx_lu_solve(cflx_lu*, int nrhs, const double* B_local, double* X_local, double* ms_out);
 /* 1 when this plan's trailing update runs on the int8 tcgen05 path (ozaki.cu), 0 for the FP64 DMMA kernel (gemm.cu) */
 int cflx_lu_uses_tcgen05(const cflx_lu*);
 /* number of kernels this plan launched since the last call (for bench.py's gpu_launches) */
@@ -152,6 +165,8 @@ int cflx_dbg_panel(int n, int v, const double* panel, int* perm_out, double* A00
                    double* ms_out);
 /* X = B * U^-1 (right, upper, non-unit; B n x v) and Y = L^-1 * R (left, lower, unit; R v x n), A00 = L\U packed */
 int cflx_dbg_trsm(int n, int v, const double* A00, const double* B, double* X_out, const double* R, double* Y_out);
+/* X = U^-1 * R (left, upper, non-unit; R v x n row-major), U = upper(A00) -- the diagonal-tile solve of cflx_lu_solve */
+int cflx_dbg_trsm_left_upper(int v, int n, const double* A00, const double* R, double* X_out);
 /* D = C - AT^T * B on the int8 tcgen05 path (error-free digit planes, ozaki.cu); K % 128 == 0, N even.  Optional test
  * outputs: digit planes [8][M][K] / [8][N][K], exponents [M] / [N].  ms_out / split_ms_out: mean device time of the GEMM
  * kernel / of the two digit-plane kernels. */
