@@ -355,6 +355,18 @@ class dbg:
         return X
 
     @staticmethod
+    def potrf_tile(A, blocked=False):
+        """Cholesky of one v x v tile (lower triangle of A referenced) by the factorisation's own tile kernels: the
+        one-CTA kernel (blocked=False) or the 128-wide blocked path (blocked=True, v in 256/384/512).
+        Returns (L, LT, info) with info = dpotrf's (1-based column of the first non-positive pivot, 0 = success)."""
+        A = np.ascontiguousarray(A, dtype=np.float64)
+        v = A.shape[0]
+        L, LT, info = np.empty((v, v)), np.empty((v, v)), ctypes.c_int()
+        check(lib().cflx_dbg_potrf_tile(v, int(bool(blocked)), A.ctypes.data, L.ctypes.data, LT.ctypes.data,
+                                        ctypes.byref(info)), "dbg_potrf_tile")
+        return L, LT, info.value
+
+    @staticmethod
     def ozaki_gemm(AT, B, C=None, reps=1, want_planes=False):
         """D = C - AT^T @ B on the int8 tcgen05 path.  Returns dict(D, ms, split_ms[, pa, pb, ea, eb])."""
         AT = np.ascontiguousarray(AT, dtype=np.float64)

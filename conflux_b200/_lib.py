@@ -25,7 +25,7 @@ SYMBOLS = [
     "cflx_lu_get_permutation", "cflx_lu_residual", "cflx_lu_validate", "cflx_lu_solve", "cflx_lu_launch_count", "cflx_lu_uses_tcgen05", "cflx_lu_set_profiling", "cflx_lu_phase_ms", "cflx_lu_timeline",
     "cflx_lu_set_kernel_timing", "cflx_lu_trailing_stats", "cflx_lu_destroy", "cflx_chol_auto_grid", "cflx_chol_auto_tile", "cflx_chol_dims", "cflx_chol_init_matrix_host",
     "cflx_chol_create", "cflx_chol_info", "cflx_chol_set_local", "cflx_chol_factor", "cflx_chol_get_local", "cflx_chol_validate",
-    "cflx_chol_launch_count", "cflx_chol_destroy", "cflx_dbg_gemm_tn", "cflx_dbg_panel", "cflx_dbg_trsm", "cflx_dbg_trsm_left_upper", "cflx_dbg_push_pivots", "cflx_dbg_ozaki_gemm", "cflx_dbg_umma_peak", "cflx_dbg_last_panel_cycles", "cflx_dbg_fp64_peak", "cflx_dbg_fp64_peak_ex",
+    "cflx_chol_launch_count", "cflx_chol_destroy", "cflx_dbg_gemm_tn", "cflx_dbg_panel", "cflx_dbg_trsm", "cflx_dbg_trsm_left_upper", "cflx_dbg_potrf_tile", "cflx_dbg_push_pivots", "cflx_dbg_ozaki_gemm", "cflx_dbg_umma_peak", "cflx_dbg_last_panel_cycles", "cflx_dbg_fp64_peak", "cflx_dbg_fp64_peak_ex",
 ]
 
 
@@ -101,6 +101,7 @@ def lib():
         L.cflx_dbg_panel.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 4 + [ctypes.c_int, c_double_p]
         L.cflx_dbg_trsm.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 5
         L.cflx_dbg_trsm_left_upper.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 3
+        L.cflx_dbg_potrf_tile.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 4
         L.cflx_dbg_push_pivots.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int,
                                            ctypes.c_void_p, ctypes.c_void_p]
         L.cflx_dbg_ozaki_gemm.argtypes = [ctypes.c_int] * 3 + [ctypes.c_void_p] * 8 + [ctypes.c_int, c_double_p, c_double_p]

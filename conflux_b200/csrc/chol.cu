@@ -18,6 +18,7 @@
 // in the LU path, so the TRSM and the rank-v update run on the same FP64 tensor-core GEMM (gemm.cu) on long contiguous
 // operands instead of v x v tile calls.  The "A10 -> A01 representative" exchange of the reference (every rank needs the
 // panel rows of its tile rows AND of its tile columns) is one grouped broadcast of the Px panel pieces to all ranks.
+#include <climits>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -49,10 +50,12 @@ namespace {
 // Cholesky of one v x v tile (row-major, lower triangle referenced) by ONE CTA: right-looking, 32-column blocks.
 //   D   in: the tile; out: L in the lower triangle, zeros above
 //   UT  out: L^T (upper triangular, row-major) -- the operand of the panel TRSM and what is broadcast
-// info[0] = 1 + index of the first non-positive pivot (0 = success), like LAPACK's dpotrf.
+// info[0] = global column + 1 of the first non-positive pivot, like LAPACK's dpotrf on the whole matrix.  A kernel writes
+// it only while it is still 0: after a failure NaN reaches every later block and tile, and on one stream the first
+// failure must win.
 constexpr int PB = 32;
 // D: v x v window (leading dimension ldd) of the tile, UT: the same window of L^T (leading dimension ldu); Uc (optional): a
-// contiguous v x v copy of the factored block's L^T; col_off: column of the window inside the whole tile (for *info)
+// contiguous v x v copy of the factored block's L^T; col_off: global column of the window's first column (for *info)
 __global__ void __launch_bounds__(1024) potrf_tile_kernel(double* __restrict__ D, int v, int ldd, double* __restrict__ UT, int ldu,
                                                           double* __restrict__ Uc, int* __restrict__ info, int col_off) {
     extern __shared__ double sm[];
@@ -168,7 +171,7 @@ __global__ void __launch_bounds__(1024) potrf_tile_kernel(double* __restrict__ D
         __syncthreads();
         for (int e = t; e < v * v; e += blockDim.x) Uc[e] = UT[(size_t)(e / v) * ldu + e % v];
     }
-    if (t == 0 && s_bad) info[0] = s_bad;
+    if (t == 0 && s_bad && info[0] == 0) info[0] = s_bad;
 }
 
 // Cholesky of ONE 128 x 128 diagonal block held entirely in shared memory (the building block of potrf_tile): all 512
@@ -248,7 +251,7 @@ __global__ void __launch_bounds__(QTHREADS) potrf128_kernel(double* __restrict__
         UT[(size_t)r * ldu + c] = lt;
         Uc[e] = lt;
     }
-    if (t == 0 && s_bad) info[0] = s_bad;
+    if (t == 0 && s_bad && info[0] == 0) info[0] = s_bad;   // the first failure wins (see potrf_tile_kernel)
 }
 
 // zeros above the diagonal of D (= L) and below the diagonal of UT (= L^T)
@@ -482,15 +485,27 @@ int broadcast_and_update(cflx_chol* ch, int t, int jmin, bool below_only, double
 // factorisation), so the tile is itself factored in 128-wide block columns: the 128 x 128 diagonal block on one CTA, the
 // block column below it by ONE GEMM with the inverted block, the trailing part of the tile by one rank-128 GEMM -- both on
 // the whole GPU (FP64 DMMA kernel).  Tiles that are not a multiple of 128 (tests) keep the one-CTA kernel.
-int potrf_tile(cflx_chol* ch, size_t psm, cudaStream_t s) {
-    const int v = ch->v;
-    constexpr int QB = 128;
-    if (v % QB != 0 || v < 2 * QB || ch->Q == nullptr) {
-        potrf_tile_kernel<<<1, 1024, psm, s>>>(ch->D, v, v, ch->A00, v, nullptr, ch->info + 1, 0);
+//   D [v][v] in: the tile, out: L (zeros above the diagonal);  UT [v][v] out: L^T;  Q: scratch of the blocked path
+//   (potrf_tile_scratch(v) doubles; nullptr selects the one-CTA kernel);  info: see potrf_tile_kernel;  col0: global column
+//   of the tile's first column.  Adds its kernel launches to *launches.  The factorisation and cflx_dbg_potrf_tile both
+//   run this.
+constexpr int QB = 128;
+size_t potrf_tile_smem(int v) { return ((size_t)PB * (PB + 1) + (size_t)v * (PB + 1)) * sizeof(double); }
+size_t potrf_tile_scratch(int v) { return (size_t)3 * QB * QB + (size_t)2 * QB * v; }
+bool potrf_tile_blocked(int v) { return v % QB == 0 && v >= 2 * QB; }
+int potrf_tile_setup(int v) {   // shared memory limits of both kernels (per device)
+    CFLX_CUDA(cudaFuncSetAttribute(potrf_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)potrf_tile_smem(v)));
+    CFLX_CUDA(cudaFuncSetAttribute(potrf128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(QBK * QPITCH * sizeof(double))));
+    return CFLX_OK;
+}
+int potrf_tile(int v, double* D, double* UT, double* Q, int* info, int col0, cudaStream_t s, int64_t* launches) {
+    if (!potrf_tile_blocked(v) || Q == nullptr) {
+        potrf_tile_kernel<<<1, 1024, potrf_tile_smem(v), s>>>(D, v, v, UT, v, nullptr, info, col0);
         CFLX_CUDA(cudaGetLastError());
+        *launches += 1;
         return CFLX_OK;
     }
-    double* U128 = ch->Q;                      // [QB][QB]  L_d^T of the current diagonal block, contiguous
+    double* U128 = Q;                          // [QB][QB]  L_d^T of the current diagonal block, contiguous
     double* Ui = U128 + QB * QB;               // [QB][QB]  its inverse
     double* Li = Ui + QB * QB;                 // [QB][QB]  (unit-lower companion of launch_diag_inverses, unused)
     double* XT0 = Li + QB * QB;                // [QB][v]   block column below the diagonal block, transposed
@@ -498,31 +513,31 @@ int potrf_tile(cflx_chol* ch, size_t psm, cudaStream_t s) {
     static_assert(QB == QBK, "block width of the tile Cholesky");
     for (int jb = 0; jb < v; jb += QB) {
         const int m = v - jb - QB;
-        potrf128_kernel<<<1, QTHREADS, QBK * QPITCH * sizeof(double), s>>>(ch->D + (size_t)jb * v + jb, v, ch->A00 + (size_t)jb * v + jb, v,
-                                                                        U128, ch->info + 1, jb);
+        potrf128_kernel<<<1, QTHREADS, QBK * QPITCH * sizeof(double), s>>>(D + (size_t)jb * v + jb, v, UT + (size_t)jb * v + jb, v, U128,
+                                                                        info, col0 + jb);
         CFLX_CUDA(cudaGetLastError());
-        ch->launches++;
+        *launches += 1;
         if (m <= 0) break;
         const int64_t ldx = m;
-        CFLX_TRY(launch_extract_panel_T(ch->D, v, jb + QB, jb, m, QB, XT0, ldx, s));
+        CFLX_TRY(launch_extract_panel_T(D, v, jb + QB, jb, m, QB, XT0, ldx, s));
         CFLX_TRY(launch_diag_inverses(U128, QB, QB, Ui, Li, s));
         CFLX_TRY(trsm_right_upper_T(U128, Ui, QB, QB, XT0, XT, ldx, m, s));          // X^T = L_d^-1 P^T
-        CFLX_TRY(launch_store_panel_T(ch->D, v, jb + QB, jb, m, QB, XT, ldx, s));
-        CFLX_CUDA(cudaMemcpy2DAsync(ch->A00 + (size_t)jb * v + jb + QB, (size_t)v * sizeof(double), XT, ldx * sizeof(double),
+        CFLX_TRY(launch_store_panel_T(D, v, jb + QB, jb, m, QB, XT, ldx, s));
+        CFLX_CUDA(cudaMemcpy2DAsync(UT + (size_t)jb * v + jb + QB, (size_t)v * sizeof(double), XT, ldx * sizeof(double),
                                     (size_t)m * sizeof(double), QB, cudaMemcpyDeviceToDevice, s));
         GemmArgs g{};                                                                 // T -= X X^T
         g.M = m; g.N = m; g.K = QB;
         g.AT = XT; g.ldat = ldx;
         g.B = XT; g.ldb = ldx;
-        g.C = ch->D + (size_t)(jb + QB) * v + jb + QB; g.ldc = v;
-        g.D = ch->D + (size_t)(jb + QB) * v + jb + QB; g.ldd = v;
+        g.C = D + (size_t)(jb + QB) * v + jb + QB; g.ldc = v;
+        g.D = D + (size_t)(jb + QB) * v + jb + QB; g.ldd = v;
         g.alpha = -1.0; g.beta = 1.0;
         CFLX_TRY(launch_gemm_tn(g, s));
-        ch->launches += 6;
+        *launches += 6;
     }
-    tri_clean_kernel<<<(v * v + 255) / 256, 256, 0, s>>>(ch->D, ch->A00, v);
+    tri_clean_kernel<<<(v * v + 255) / 256, 256, 0, s>>>(D, UT, v);
     CFLX_CUDA(cudaGetLastError());
-    ch->launches++;
+    *launches += 1;
     return CFLX_OK;
 }
 
@@ -538,7 +553,6 @@ int panel_step(cflx_chol* ch, int k, cudaStream_t s) {
     const int64_t ld1 = piece_ld(ch, k + 1, pi);                 // rows strictly below tile k (what is broadcast)
     const bool on_col = (pj == pjk);
     const bool owner = on_col && pi == pik && pk == 0;
-    const size_t psm = ((size_t)PB * (PB + 1) + (size_t)v * (PB + 1)) * sizeof(double);
     // (4 of the previous step) tile column k summed over the z layers                  Cholesky.cpp:580-612
     if (on_col && n0 > 0) {
         CFLX_TRY(launch_extract_panel_T(ch->A11, Nl, row0, loff, n0, v, ch->PT, ld, s));
@@ -548,10 +562,10 @@ int panel_step(cflx_chol* ch, int k, cudaStream_t s) {
     // (1) Cholesky of the diagonal tile                                                 Cholesky.cpp:188-193
     if (owner) {
         tile_from_panel_kernel<<<(v * v + 255) / 256, 256, 0, s>>>(ch->PT, ld, v, ch->D);
-        CFLX_TRY(potrf_tile(ch, psm, s));
+        CFLX_TRY(potrf_tile(v, ch->D, ch->A00, ch->Q, ch->info + 1, k * v, s, &ch->launches));
         tile_store_kernel<<<(v * v + 255) / 256, 256, 0, s>>>(ch->D, v, ch->A11 + (int64_t)row0 * Nl + loff, Nl);
         CFLX_CUDA(cudaGetLastError());
-        ch->launches += 3;
+        ch->launches += 2;
     }
     if (k == ch->Kappa - 1) return CFLX_OK;
     // L_kk^T to the ranks that hold the tile column (layer 0)                           Cholesky.cpp:680-690
@@ -691,7 +705,7 @@ int cflx_chol_create(cflx_comm* c, int N, int v, int Px, int Py, int Pz, cflx_ch
     ALLOC(ch->G, 2 * (size_t)Px * v * ch->ldp); ALLOC(ch->Bc, 2 * (size_t)v * ch->ldb);
     ALLOC(ch->D, vv); ALLOC(ch->A00, vv); ALLOC(ch->Uinv, vv); ALLOC(ch->LinvT, vv); ALLOC(ch->acc, 4);
     ALLOC(ch->info, 4);
-    if (v % 128 == 0 && v >= 256) ALLOC(ch->Q, (size_t)3 * 128 * 128 + (size_t)2 * 128 * v);
+    if (potrf_tile_blocked(v)) ALLOC(ch->Q, potrf_tile_scratch(v));
 #undef ALLOC
     cudaMemsetAsync(ch->PT, 0, (size_t)v * ch->ldp * sizeof(double), c->stream);
     cudaMemsetAsync(ch->LT, 0, (size_t)v * ch->ldp * sizeof(double), c->stream);
@@ -717,9 +731,7 @@ int cflx_chol_create(cflx_comm* c, int N, int v, int Px, int Py, int Pz, cflx_ch
                 cudaEventCreateWithFlags(&ch->ev_panel[i], cudaEventDisableTiming) != cudaSuccess)
                 return fail(CFLX_ERR_CUDA);
     }
-    const size_t psm = ((size_t)PB * (PB + 1) + (size_t)v * (PB + 1)) * sizeof(double);
-    if (cudaFuncSetAttribute(potrf_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm) != cudaSuccess) return fail(CFLX_ERR_CUDA);
-    if (cudaFuncSetAttribute(potrf128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(QBK * QPITCH * sizeof(double))) != cudaSuccess) return fail(CFLX_ERR_CUDA);
+    if ((rc = potrf_tile_setup(v))) return fail(rc);
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) return fail(CFLX_ERR_CUDA);
     *out = ch;
     return CFLX_OK;
@@ -792,10 +804,21 @@ int cflx_chol_factor(cflx_chol* ch, double* ms_out) {
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     CFLX_CUDA(cudaGetLastError());
+    // Only the owner of a diagonal tile sees its pivots: the first failing column (the smallest nonzero info) is agreed on
+    // by every rank, so that the collective call returns the same answer everywhere.
     int h[4] = {0, 0, 0, 0};
     CFLX_CUDA(cudaMemcpy(h, ch->info, sizeof(h), cudaMemcpyDeviceToHost));
+    if (ch->P > 1) {
+        const int mine = h[1] != 0 ? h[1] : INT_MAX;
+        CFLX_CUDA(cudaMemcpyAsync(ch->info + 2, &mine, sizeof(int), cudaMemcpyHostToDevice, s));
+        CFLX_NCCL(ncclAllReduce(ch->info + 2, ch->info + 2, 1, ncclInt32, ncclMin, c->world, s));
+        CFLX_CUDA(cudaMemcpyAsync(&h[2], ch->info + 2, sizeof(int), cudaMemcpyDeviceToHost, s));
+        CFLX_CUDA(cudaStreamSynchronize(s));
+        h[1] = h[2] == INT_MAX ? 0 : h[2];
+    }
     if (h[1] != 0) {
-        set_last_error("cholesky: the matrix is not positive definite (a diagonal tile failed at column %d)", h[1]);
+        set_last_error("cholesky: the matrix is not positive definite (the leading minor of order %d is not positive: "
+                       "column %d, like dpotrf's info)", h[1], h[1]);
         return CFLX_ERR_STATE;
     }
     if (ms_out) *ms_out = ms;
@@ -891,5 +914,45 @@ int cflx_chol_launch_count(cflx_chol* ch, int64_t* count_out, int reset) {
 }
 
 void cflx_chol_destroy(cflx_chol* ch) { free_chol(ch); }
+
+// The diagonal-tile Cholesky of cflx_chol_factor alone (the same potrf_tile), on the current device: A v x v row-major (lower
+// triangle referenced), L_out = L with zeros above the diagonal, LT_out = L^T, info_out as dpotrf.  L^T starts as NaN, so a
+// value the kernels never write shows up.
+int cflx_dbg_potrf_tile(int v, int blocked, const double* A, double* L_out, double* LT_out, int* info_out) {
+    if (v <= 0 || v % 4 != 0 || v > 512 || (blocked != 0 && blocked != 1) || !A || !L_out || !LT_out || !info_out)
+        return CFLX_ERR_ARG;
+    if (blocked && !potrf_tile_blocked(v)) {
+        set_last_error("blocked tile Cholesky needs v %% 128 == 0 and v >= 256 (v=%d)", v);
+        return CFLX_ERR_UNSUPPORTED;
+    }
+    int n = 0;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
+        cudaGetLastError();
+        set_last_error("no CUDA device visible: conflux_b200 has no CPU fallback");
+        return CFLX_ERR_NO_DEVICE;
+    }
+    const size_t vv = (size_t)v * v;
+    double *D = nullptr, *UT = nullptr, *Q = nullptr;
+    int* info = nullptr;
+    int rc = dmalloc(&D, vv);
+    if (!rc) rc = dmalloc(&UT, vv);
+    if (!rc && blocked) rc = dmalloc(&Q, potrf_tile_scratch(v));
+    if (!rc) rc = dmalloc(&info, 1);
+    if (!rc) rc = gemm_tn_setup();
+    if (!rc) rc = potrf_tile_setup(v);
+    if (!rc && (cudaMemcpy(D, A, vv * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess ||
+                cudaMemset(UT, 0xff, vv * sizeof(double)) != cudaSuccess || cudaMemset(info, 0, sizeof(int)) != cudaSuccess))
+        rc = CFLX_ERR_CUDA;
+    int64_t launches = 0;
+    if (!rc) rc = potrf_tile(v, D, UT, Q, info, 0, 0, &launches);
+    if (!rc && (cudaMemcpy(L_out, D, vv * sizeof(double), cudaMemcpyDeviceToHost) != cudaSuccess ||
+                cudaMemcpy(LT_out, UT, vv * sizeof(double), cudaMemcpyDeviceToHost) != cudaSuccess ||
+                cudaMemcpy(info_out, info, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess)) {
+        set_last_error("tile Cholesky failed: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = CFLX_ERR_CUDA;
+    }
+    for (void* p : {(void*)D, (void*)UT, (void*)Q, (void*)info}) cudaFree(p);
+    return rc;
+}
 
 }  // extern "C"

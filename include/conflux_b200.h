@@ -148,7 +148,9 @@ int cflx_chol_create(cflx_comm*, int N, int v, int Px, int Py, int Pz, cflx_chol
 /* info_out[16] = {N, v, Kappa, Ml, Nl, v / Pz, P, Px, Py, Pz, pi, pj, pk, rank, 0, 0} */
 int cflx_chol_info(const cflx_chol*, int* info_out);
 int cflx_chol_set_local(cflx_chol*, const double* host_local);
-/* COLLECTIVE.  ms_out = device time of the factorisation loop (the region the reference's miniapp times). */
+/* COLLECTIVE.  ms_out = device time of the factorisation loop (the region the reference's miniapp times).  A matrix that
+ * is not positive definite returns CFLX_ERR_STATE on EVERY rank, and cflx_last_error() names the first failing column,
+ * 1-based, like LAPACK dpotrf's info ("... not positive definite ... column <c> ..."); the factor is then not available. */
 int cflx_chol_factor(cflx_chol*, double* ms_out);
 int cflx_chol_get_local(cflx_chol*, double* L_host);
 /* COLLECTIVE.  ||A - L L^T||_F over the lower triangle, absolute and relative to ||A||_F, computed on the GPU grid. */
@@ -167,6 +169,11 @@ int cflx_dbg_panel(int n, int v, const double* panel, int* perm_out, double* A00
 int cflx_dbg_trsm(int n, int v, const double* A00, const double* B, double* X_out, const double* R, double* Y_out);
 /* X = U^-1 * R (left, upper, non-unit; R v x n row-major), U = upper(A00) -- the diagonal-tile solve of cflx_lu_solve */
 int cflx_dbg_trsm_left_upper(int v, int n, const double* A00, const double* R, double* X_out);
+/* the diagonal-tile Cholesky of cflx_chol_factor: A v x v row-major (lower triangle referenced), L_out = L (zeros above the
+ * diagonal), LT_out = L^T, info_out = dpotrf's info (1-based first non-positive pivot, 0 = success).  blocked = 0: the
+ * one-CTA kernel (v % 4 == 0, v <= 512); blocked = 1: 128-wide block columns on the GEMMs (v % 128 == 0, v >= 256), what
+ * the factorisation uses for those v. */
+int cflx_dbg_potrf_tile(int v, int blocked, const double* A, double* L_out, double* LT_out, int* info_out);
 /* D = C - AT^T * B on the int8 tcgen05 path (error-free digit planes, ozaki.cu); K % 128 == 0, N even.  Optional test
  * outputs: digit planes [8][M][K] / [8][N][K], exponents [M] / [N].  ms_out / split_ms_out: mean device time of the GEMM
  * kernel / of the two digit-plane kernels. */

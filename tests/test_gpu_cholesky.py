@@ -11,7 +11,10 @@ from tests._harness import n_gpus, run_ranks
 pytestmark = pytest.mark.gpu
 
 
-def _run(N, v, grid, A_global=None):
+def _run(N, v, grid, A_global=None, twice=False, catch=False):
+    """Factor A_global (default: the reference's generator) on the grid.  Returns (A, L, per-rank results).
+    twice: factor a second time without uploading again, L of that run in r["L2"] (assembled: r["L2g"] of rank 0).
+    catch: a ConfluxError of parallelCholesky() is returned as r["error"] on each rank (A and L are then None)."""
     P = grid[0] * grid[1] * grid[2]
     if n_gpus() < P:
         pytest.skip(f"needs {P} GPUs")
@@ -24,14 +27,27 @@ def _run(N, v, grid, A_global=None):
                     gi, gj = lti * ch.PX + ch.px, ltj * ch.PY + ch.py
                     if gi < ch.Kappa and gj < ch.Kappa:
                         ch.data[lti * v:(lti + 1) * v, ltj * v:(ltj + 1) * v] = A_global[gi * v:(gi + 1) * v, gj * v:(gj + 1) * v]
-        ms = ch.parallelCholesky()
+        try:
+            ms = ch.parallelCholesky()
+        except cb.ConfluxError as e:
+            if not catch:
+                raise
+            ch.finalize()
+            return dict(error=str(e), rank=ch.rank)
         res = dict(A=ch.data.copy(), L=ch.local_factor() if ch.pz == 0 else None, resid=ch.validate(), ms=ms, rank=ch.rank)
+        if twice:
+            ch.parallelCholesky(upload=False)
+            res["L2"] = ch.local_factor() if ch.pz == 0 else None
         ch.finalize()
         return res
 
     rs = run_ranks(P, body)
+    if any("error" in r for r in rs):
+        return None, None, rs
     A = chol_ref.assemble([r["A"] for r in rs], N, v, *grid)
     L = np.tril(chol_ref.assemble([r["L"] for r in rs], N, v, *grid))
+    if twice:
+        rs[0]["L2g"] = np.tril(chol_ref.assemble([r["L2"] for r in rs], N, v, *grid))
     return A, L, rs
 
 
